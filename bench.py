@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RTR iterations/sec on sphere2500 (BASELINE.json metric) + the Q.X SpMV roofline.
 
-    python bench.py --gpus N --steps K --warmup W          (N>1: launched by torch.distributed.run)
+    python bench.py --gpus N --steps K --warmup W [--dump-outputs DIR]   (N>1: launched by torch.distributed.run)
     python bench.py --impl reference --steps K --warmup W  (CPU restatement of the reference path)
 
 A "step" is one QuadraticOptimizer::optimize() call with the constants PGOAgent::updateX uses
@@ -52,6 +52,21 @@ def measured_peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT = 64 << 20   # bytes, all arrays of one --dump-outputs directory
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """--dump-outputs: what the timed path computed in its last step, one float64 <name>.npy per array, so that two
+    builds run with the same arguments (hence the same inputs) can be compared output for output."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def ncu_traffic(kernel: str):
@@ -253,7 +268,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, args.steps)
+    steps = args.steps
     if args.gpus > 1:
         # the multi-GPU arm's workload: sphere2500 split into MULTI_AGENTS agents, coloured RBCD; value = rounds/s
         val, dt, info = cpu_multi_agent_rounds(DATASET, MULTI_AGENTS, steps, min(args.warmup, 4))
@@ -391,6 +406,11 @@ def run_gpu_arm(args):
         e1.record()
         barrier()
         ms_total = e0.elapsed_time(e1)
+        outputs = None
+        if args.dump_outputs:
+            # the iterate and the result record of the last timed step, before the end-to-end leg overwrites them
+            rs_last = opt.fetch_result()
+            outputs = {"X": prob.download_X(), "f_opt": [rs_last.f_opt], "gradnorm_opt": [rs_last.gradnorm_opt]}
         # ---- end to end: public API, pinned host buffers, H2D + D2H inside the timed region ----
         def pinned():                       # (r, N) Fortran-ordered view of a pinned (N, r) tensor
             t = torch.empty(((d + 1) * n, RANK_R), dtype=torch.float64).pin_memory()
@@ -474,7 +494,7 @@ def run_gpu_arm(args):
             # the multi-GPU arm's workloads with all agents on this one GPU: the 1-GPU point of the scaling curve
             line["multi_agent_1gpu"] = {}
             for ds in (DATASET, "torus3D"):
-                m = measure_multi(torch, None, dp, pg, ds, MULTI_AGENTS, 0, 1, local_rank, max(K, 48), W, peak, peak_src, with_e2e=False)
+                m = measure_multi(torch, None, dp, pg, ds, MULTI_AGENTS, 0, 1, local_rank, K, W, peak, peak_src, with_e2e=False)
                 line["multi_agent_1gpu"][ds] = {k2: m[k2] for k2 in ("rounds_per_sec", "ms_per_round", "agent_steps_per_sec", "colours", "final",
                                                                      "concurrent_agents", "step_kernel_launch")}
         if not args.no_spmv:
@@ -493,12 +513,16 @@ def run_gpu_arm(args):
         if not args.no_cpu:
             _, _, info = cpu_reference_steps(2 * CYCLE, 1)
             line["cpu_baseline"] = info
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     else:
         sampler = ClockSampler(local_rank)
         if rank == 0:
             sampler.start()
-        res = measure_multi(torch, dist, dp, pg, DATASET, MULTI_AGENTS, rank, world, local_rank, K, W, peak, peak_src, with_e2e=True)
+        outputs = {} if args.dump_outputs else None
+        res = measure_multi(torch, dist, dp, pg, DATASET, MULTI_AGENTS, rank, world, local_rank, K, W, peak, peak_src, with_e2e=True,
+                            outputs=outputs)
         tor = measure_multi(torch, dist, dp, pg, "torus3D", MULTI_AGENTS, rank, world, local_rank, K, W, peak, peak_src, with_e2e=False)
         if rank == 0:
             clocks = sampler.stop()
@@ -516,13 +540,16 @@ def run_gpu_arm(args):
                                                     "roofline", "allgather_bytes_per_rank", "concurrent_agents", "step_kernel_launch")},
             })
             print(json.dumps(line))
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)      # every rank writes the iterates of its own agents
         dist.destroy_process_group()
 
 
-def measure_multi(torch, dist, dp, pg, dataset, k, rank, world, local_rank, K, W, peak, peak_src, with_e2e):
+def measure_multi(torch, dist, dp, pg, dataset, k, rank, world, local_rank, K, W, peak, peak_src, with_e2e, outputs=None):
     """K timed coloured RBCD rounds of `dataset` split into k agents spread over `world` ranks (k/world agents per GPU).
     Returns rounds/s (max over ranks of the CUDA-event time), the per-rank roofline of the k_optimize launches of rank 0,
-    and optionally the same rounds through the host-level API (host matrices in and out every round)."""
+    and optionally the same rounds through the host-level API (host matrices in and out every round).
+    outputs: if a dict, receives X_agent<a> = this rank's agents' iterates after the last timed round."""
     from dpo_b200.agent import DistributedPGO
     dev = torch.device("cuda", local_rank)
     edges, n = pg.read_g2o_file(os.path.join(ROOT, "data", dataset + ".g2o"))
@@ -596,6 +623,9 @@ def measure_multi(torch, dist, dp, pg, dataset, k, rank, world, local_rank, K, W
     with torch.cuda.stream(side):
         e1.record()
     barrier()
+    if outputs is not None:
+        for a in mine:
+            outputs[f"X_agent{a:02d}"] = run.agents[a].mProblem.download_X()
     t = torch.tensor([e0.elapsed_time(e1), float(my_steps)], dtype=torch.float64, device=dev)
     tmax, tsum = t.clone(), t.clone()
     if distributed:
@@ -632,14 +662,13 @@ def measure_multi(torch, dist, dp, pg, dataset, k, rank, world, local_rank, K, W
             cols = (run.glob[a][:, None] * dh + np.arange(dh)[None, :]).ravel()
             ag.X = np.array(X0[:, cols])
         run.round = 0
-        KE = max(50, K // 2)
         with torch.cuda.stream(side):
             for _ in range(2 * run.ncolours):
                 run.step_host()
         barrier()
         t0 = time.perf_counter()
         with torch.cuda.stream(side):
-            for i in range(KE):
+            for i in range(K):
                 if i % cyc == 0:
                     for a in mine:
                         cols = (run.glob[a][:, None] * dh + np.arange(dh)[None, :]).ravel()
@@ -652,7 +681,7 @@ def measure_multi(torch, dist, dp, pg, dataset, k, rank, world, local_rank, K, W
         if distributed:
             dist.all_reduce(te, op=dist.ReduceOp.MAX)
         h2d, d2h = run.host_bytes_per_step()
-        out["e2e"] = {"value": KE / float(te[0]), "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "rounds": KE,
+        out["e2e"] = {"value": K / float(te[0]), "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "rounds": K,
                       "api": "DistributedPGO.step_host(): per round every local agent's X from pinned host memory (H2D), device-side "
                              "exchange (pack -> all-gather -> G rebuild), RTR step of the active agents, their X back to the host (D2H)"
                              + ("; 3 C calls per round (dpgo_agents_host_io_async x2, dpgo_agents_round_async), each replayed as a CUDA graph"
@@ -674,7 +703,14 @@ def main():
     ap.add_argument("--no-sweep", action="store_true", help="N = 1: skip the SpMV size sweep")
     ap.add_argument("--precond", default="sparse", choices=["sparse", "dense"],
                     help="exact preconditioner implementation: nested-dissection block solve (default) or the dense inverse (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float64): "
+                         "N = 1: X (the iterate, r x (d+1)n), f_opt, gradnorm_opt; N > 1: X_agent<a> per agent")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -109,8 +109,9 @@ def build_host(force: bool = False) -> str:
     return HOST_LIB
 
 
-def build_cpp_program(sources, output, defines=(), extra_includes=()):
-    """Compile a C++ program against libDPGO.so (used for the reference's unchanged examples/tests and ours)."""
+def build_cpp_program(sources, output, defines=(), extra_includes=(), rpath=None):
+    """Compile a C++ program against libDPGO.so (used for the reference's unchanged examples/tests and ours).
+    rpath: where the program looks for the libraries at run time (default: this tree's lib/ by absolute path)."""
     build_host()
     os.makedirs(os.path.dirname(output), exist_ok=True)
     cmd = [CXX] + CXXFLAGS
@@ -118,7 +119,8 @@ def build_cpp_program(sources, output, defines=(), extra_includes=()):
         cmd += ["-I", inc]
     for dname in defines:
         cmd += ["-D" + dname]
-    cmd += list(sources) + ["-o", output, "-L", LIBDIR, "-lDPGO", "-ldpgo_b200", "-lnccl", "-Wl,-rpath," + LIBDIR, "-lpthread"]
+    cmd += list(sources) + ["-o", output, "-L", LIBDIR, "-lDPGO", "-ldpgo_b200", "-lnccl", "-Wl,-rpath," + (rpath or LIBDIR),
+                            "-lpthread"]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError(f"compile failed for {sources}:\n{res.stderr[-4000:]}")
@@ -139,34 +141,8 @@ def build_examples():
     return out
 
 
-REFERENCE = "/root/reference"
-REF_BUILD = os.path.join(HERE, "..", "build", "ref")
-
-
-def build_reference_drivers():
-    """Compile the reference's OWN example drivers and gtest files, unchanged, from where they lie under
-    /root/reference, against the B200 host library ("link unchanged").  Only possible in the container that has
-    the reference mounted; the binaries land in build/ref/ and travel to the GPU box."""
-    if not os.path.isdir(REFERENCE):
-        return []
-    out = []
-    bindir = os.path.abspath(os.path.join(REF_BUILD, "bin"))
-    for name in ("MultiRobotExample", "SingleRobotExample"):
-        src = os.path.join(REFERENCE, "examples", name + ".cpp")
-        out.append(build_cpp_program([src], os.path.join(bindir, name)))
-    gtest_inc = os.path.join(INCLUDE, "gtest_shim")
-    tests = [os.path.join(REFERENCE, "tests", f) for f in
-             ("testConstruction.cpp", "testLineGraph.cpp", "testTriangleGraph.cpp", "testOptimizationThread.cpp")]
-    main_cpp = os.path.join(os.path.abspath(REF_BUILD), "gtest_main.cpp")
-    os.makedirs(os.path.dirname(main_cpp), exist_ok=True)
-    with open(main_cpp, "w") as fh:
-        fh.write('#define GTEST_SHIM_MAIN\n#include "gtest/gtest.h"\n')
-    out.append(build_cpp_program(tests + [main_cpp], os.path.join(bindir, "testDPGO"), extra_includes=[gtest_inc]))
-    return out
-
-
 if __name__ == "__main__":
     print(build_library(force="--force" in sys.argv, verbose=True))
     print(build_host(force="--force" in sys.argv))
-    for b in build_examples() + build_reference_drivers():
+    for b in build_examples():
         print(b)

@@ -1,9 +1,13 @@
 """bench.py contract (CPU side): the reference arm runs without a GPU and prints ONE JSON line with the keys the
-driver reads; the product arm must refuse to run without a CUDA device instead of falling back to the CPU."""
+driver reads; the product arm must refuse to run without a CUDA device instead of falling back to the CPU.  On the
+GPU: --dump-outputs writes what the last timed step computed."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -39,3 +43,26 @@ def test_product_arm_fails_loudly_without_gpu():
     out = run_bench("--steps", "1", "--warmup", "1", "--no-cpu", "--no-spmv")
     assert out.returncode != 0
     assert "{\"metric\"" not in out.stdout                   # no bench line from a CPU fallback
+
+
+def test_steps_must_be_positive():
+    out = run_bench("--impl", "reference", "--steps", "0", "--warmup", "1")
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_step(tmp_path):
+    """--steps 2: the last timed step is step 1 of the cycle from the initial point, the same step as trajectory[1]."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--no-cpu",
+                          "--no-spmv", "--no-multi", "--dump-outputs", str(tmp_path)], cwd=ROOT, capture_output=True,
+                         text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([ln for ln in out.stdout.splitlines() if ln.strip().startswith("{")][-1])
+    assert d["steps"] == 2
+    assert sorted(os.listdir(tmp_path)) == ["X.npy", "f_opt.npy", "gradnorm_opt.npy"]
+    X = np.load(os.path.join(tmp_path, "X.npy"))
+    assert X.dtype == np.float64 and X.shape == (5, 4 * 2500) and np.all(np.isfinite(X))
+    f = np.load(os.path.join(tmp_path, "f_opt.npy"))
+    g = np.load(os.path.join(tmp_path, "gradnorm_opt.npy"))
+    assert abs(f[0] - d["trajectory"][1]["f"]) <= 1e-12 * abs(f[0])
+    assert abs(g[0] - d["trajectory"][1]["gradnorm"]) <= 1e-9 * abs(g[0])

@@ -1,6 +1,6 @@
-"""The reference's OWN example drivers and gtest files, compiled UNCHANGED from /root/reference against the B200
-host library (include/DPGO + libDPGO.so + libdpgo_b200.so) by dpo_b200.build.build_reference_drivers(), run on the GPU.
-The binaries are built in the container that has the reference mounted and travel to the GPU box in build/ref/."""
+"""The reference's OWN example drivers and gtest files, compiled UNCHANGED against the B200 host library
+(include/DPGO + libDPGO.so + libdpgo_b200.so) by oracle/build_ref.py, run on the GPU.  The binaries are built where
+a checkout of the reference exists and are carried with the tree in oracle/_ref/."""
 import os
 import re
 import subprocess
@@ -11,13 +11,13 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BIN = os.path.join(ROOT, "build", "ref", "bin")
+BIN = os.path.join(ROOT, "oracle", "_ref", "bin")
 
 
 def need(name):
     path = os.path.join(BIN, name)
     if not os.path.exists(path):
-        pytest.skip(f"{path} not built (needs /root/reference at build time)")
+        pytest.skip(f"{path} not built (needs a checkout of the reference at build time, see oracle/build_ref.py)")
     return path
 
 
@@ -45,11 +45,13 @@ def test_multi_robot_example_reproduces_shipped_trace(tmp_path):
     """ref examples/MultiRobotExample.cpp main() is hard-wired to compute(5, "torus3D", false) and writes
     ../../result/graph/NPtorus3D.txt; the reference ships that very file (first 400 lines in tests/golden/)."""
     exe = need("MultiRobotExample")
-    os.makedirs(os.path.join(ROOT, "result", "graph"), exist_ok=True)
-    out = os.path.join(ROOT, "result", "graph", "NPtorus3D.txt")
-    if os.path.exists(out):
-        os.remove(out)
-    res = subprocess.run([exe], cwd=os.path.join(ROOT, "build", "ref"), capture_output=True, text=True, timeout=1800)
+    # the driver reads ../../data/ and writes ../../result/graph/ relative to its working directory
+    cwd = tmp_path / "run" / "bin"
+    cwd.mkdir(parents=True)
+    (tmp_path / "data").symlink_to(os.path.join(ROOT, "data"))
+    (tmp_path / "result" / "graph").mkdir(parents=True)
+    out = str(tmp_path / "result" / "graph" / "NPtorus3D.txt")
+    res = subprocess.run([exe], cwd=str(cwd), capture_output=True, text=True, timeout=1800)
     print(res.stdout[-1500:], res.stderr[-1500:])
     assert res.returncode == 0
     got = np.loadtxt(out, delimiter=",")
